@@ -6,6 +6,9 @@ A step = one batch of IMAGES_PER_STEP synthetic images, each through one esac.fo
 refine), exactly as the reference's callers loop over a test set with batch size 1 (test_esac.py:137-205).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          this repository's CUDA path
+  python bench.py ... --dump-outputs DIR                       also write what the timed path returned for the images of
+                                                               its last step: DIR/poses.npy [32, 4, 4] float32 (outPose) and
+                                                               DIR/experts.npy [32] float64 (the returned expert index)
   python bench.py --impl reference ...                         the reference's CPU path on the host cores: oracle/_ref (the
                                                                reference's own esac.cpp compiled against the cv2-backed OpenCV
                                                                stand-in), or the cv2 oracle port where _ref is not built
@@ -143,10 +146,7 @@ def run_reference(args, rank: int, world: int):
     from esac_b200.synth import make_scene
     sc = make_scene(E=E_PER_GPU, H=H, W=W, M=HYPS_PER_EXPERT, sub=SUB, seed=0, per_expert=True, active_only=False)
     take = min(max(4 * cores, 64), E_PER_GPU * HYPS_PER_EXPERT)
-    # a step costs seconds of CPU time and the metric is a rate: the number of steps actually run is capped so that the arm
-    # ends within minutes whatever K the driver passes; both counts are reported
-    warm_run = min(args.warmup, 1)
-    steps_run = max(1, min(args.steps, 6))
+    warm_run, steps_run = args.warmup, args.steps
     for _ in range(warm_run):
         cpu_sample(sc, take, 1)
     t0 = time.perf_counter()
@@ -296,11 +296,17 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the poses and expert indices of the last timed step's images to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
         run_reference(args, rank, world)
         return
 
@@ -331,6 +337,9 @@ def main():
     p_coords = [torch.from_numpy(s.coords) for s in scenes]     # ordinary (pageable) host tensors
     p_assign = [torch.from_numpy(s.assign) for s in scenes]
     d_out = torch.zeros(4, 4, device=dev)
+    # device-resident timed path: image p of a step writes its own 4x4 view, so the last step's poses can be dumped
+    d_poses = torch.zeros(IMAGES_PER_STEP, 4, 4, device=dev)
+    d_pose_views = list(d_poses.unbind(0))
     h_out = torch.zeros(4, 4).pin_memory()
     p_out = torch.zeros(4, 4)
     # input preparation, not a step: the first transfers out of freshly pinned pages run at a fraction of the steady PCIe rate
@@ -347,8 +356,9 @@ def main():
 
     def forward_once(i, mode: str):
         j = i % N_SCENES
-        co, asg, out = {"device": (d_coords, d_assign, d_out), "pinned": (h_coords, h_assign, h_out),
-                        "pageable": (p_coords, p_assign, p_out)}[mode]
+        co, asg, outs = {"device": (d_coords, d_assign, d_pose_views), "pinned": (h_coords, h_assign, [h_out]),
+                         "pageable": (p_coords, p_assign, [p_out])}[mode]
+        out = outs[i % len(outs)]
         if world == 1:
             return esac.forward(co[j], asg[j], out, *params)
         return sharded.forward_sharded(co[j], asg[j], out, params, expert_offset=rank * E_PER_GPU, hyp_offset=rank * M_local,
@@ -364,9 +374,10 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         acc = {s: 0.0 for s in STAGES}
         launches = score_launches = 0
+        experts = [None] * IMAGES_PER_STEP  # k starts at a multiple of IMAGES_PER_STEP: slot p = image p of a step
         e0.record()
         for _ in range(steps * IMAGES_PER_STEP):
-            forward_once(k, mode); k += 1
+            experts[k % IMAGES_PER_STEP] = forward_once(k, mode); k += 1
             st = ctx.stats()
             for s in STAGES:
                 acc[s] += st[s]
@@ -382,15 +393,16 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
         n = steps * IMAGES_PER_STEP
-        return ms, {s: acc[s] / n for s in STAGES}, launches, score_launches, ctx.stats()
+        return ms, {s: acc[s] / n for s in STAGES}, launches, score_launches, ctx.stats(), experts
 
     sampler = ClockSampler(local_rank)
     sampler.start()
-    ms, stages, launches, score_launches, last = timed("device", args.steps, args.warmup)
+    ms, stages, launches, score_launches, last, last_experts = timed("device", args.steps, args.warmup)
     clocks = sampler.stop()
-    ms_e2e, stages_e2e, _, _, _ = timed("pinned", args.steps, args.warmup)
+    last_poses = d_poses.cpu().numpy()
+    ms_e2e, stages_e2e, _, _, _, _ = timed("pinned", args.steps, args.warmup)
     steps_pg = max(1, args.steps // 4)
-    ms_pg, _, _, _, _ = timed("pageable", steps_pg, 1)
+    ms_pg, _, _, _, _, _ = timed("pageable", steps_pg, 1)
 
     # per-rank stage timers (CUDA events inside the library, read after each call's single synchronisation): max / mean over ranks
     stage_table = None
@@ -495,6 +507,11 @@ def main():
                 "stages_ms_per_forward": stages, "stages_ms_per_forward_e2e": stages_e2e, "stages_over_ranks": stage_table,
                 "score_launch": {"ppt": last["score_ppt"], "grid": last["score_grid"], "refine_group": last["refine_group"]},
                 "configs": configs}
+        if args.dump_outputs:
+            d = Path(args.dump_outputs)
+            d.mkdir(parents=True, exist_ok=True)
+            np.save(d / "poses.npy", last_poses.astype(np.float32))
+            np.save(d / "experts.npy", np.array(last_experts, np.float64))
         if world == 1 and not args.no_cpu_baseline:
             cores = os.cpu_count() or 1
             take = min(max(4 * cores, 64), M_local)
