@@ -82,6 +82,8 @@ def load_library() -> C.CDLL:
     lib.esacb200_assign_hypotheses.restype = i32
     lib.esacb200_reproj_loss.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp, vp, f32, f32, f32, i32, f32, f32, f32, vp]
     lib.esacb200_reproj_loss.restype = i32
+    lib.esacb200_init_loss.argtypes = [vp, i32, vp, i32, i32, vp, i32, i32, vp, f32, vp, vp]
+    lib.esacb200_init_loss.restype = i32
     lib.esacb200_backward_sharded.argtypes = ([vp, vp, vp, i32, i32, i32, vp, i64, i32, vp, f32, f32, f32] + cam +
                                                [EXCHANGE_FN, vp, C.POINTER(f64)])
     lib.esacb200_backward_sharded.restype = i32
@@ -598,6 +600,46 @@ def reproj_loss(prediction, gtPoses, focalLength, padX, padY, cutLoss, subSampli
     if og:
         og.finish()
     return [float(v) for v in losses]
+
+
+def init_loss(prediction, gtCoords, cutLoss, outGradients=None):
+    """The scene-coordinate loss of init_expert.py:112-130 for a batch of images.  prediction [B,3,h,w] or [3,h,w] float32,
+    gtCoords float32 of the same rank and batch; heights and widths may differ by one (both are cropped to the common
+    top-left region, util.assert_size), by more is a RuntimeError.  Target cells whose three components are all zero do not
+    count.  Returns [(loss, count)] per image: loss = robust sum / count (NaN for an image without a valid cell, as in the
+    reference), count = number of valid cells.  outGradients (prediction's shape, float32) or None receives, overwritten,
+    d(robust sum of image b) / d prediction -- the gradient of the per-image SUM; multiply image b by 1/count_b for the
+    gradient of its loss (autograd.init_loss does).  CPU, CUDA tensors or numpy arrays; CUDA work runs on torch's current
+    stream."""
+    for t, what in ((prediction, "prediction"), (gtCoords, "gtCoords")):
+        have = _dtype_name(t)
+        if have != "Float":
+            raise RuntimeError(f"expected scalar type Float but found {have} ({what})")
+    ps, gs = tuple(int(v) for v in prediction.shape), tuple(int(v) for v in gtCoords.shape)
+    if len(ps) not in (3, 4) or len(gs) != len(ps):
+        raise RuntimeError(f"prediction and gtCoords must both be [3,h,w] or [B,3,h,w] (got {list(ps)} and {list(gs)})")
+    if len(ps) == 3:
+        ps, gs = (1,) + ps, (1,) + gs
+    if ps[1] != 3 or gs[1] != 3:
+        raise RuntimeError(f"prediction and gtCoords need 3 channels (got {ps[1]} and {gs[1]})")
+    if ps[0] != gs[0]:
+        raise RuntimeError(f"batch sizes differ: prediction {ps[0]}, gtCoords {gs[0]}")
+    B = ps[0]
+    pr = _Arg(prediction)
+    gt = _Arg(gtCoords)
+    og = None
+    if outGradients is not None:
+        if _dtype_name(outGradients) != "Float" or tuple(outGradients.shape) != tuple(prediction.shape):
+            raise RuntimeError("outGradients must be float32 of prediction's shape")
+        og = _Arg(outGradients, writable=True)
+    ctx = _pick_ctx(pr.device, gt.device, og.device if og else None)
+    sums = np.zeros(B, np.float64)
+    counts = np.zeros(B, np.int64)
+    ctx.check(ctx.lib.esacb200_init_loss(ctx.handle, B, pr.ptr, ps[2], ps[3], gt.ptr, gs[2], gs[3], og.ptr if og else None,
+                                         float(cutLoss), sums.ctypes.data, counts.ctypes.data))
+    if og:
+        og.finish()
+    return [(float(s) / int(c) if c else float("nan"), int(c)) for s, c in zip(sums, counts)]
 
 
 def nccl_unique_id() -> bytes:

@@ -73,3 +73,32 @@ def reproj_loss(prediction, gt_poses, focal_length, pad_x, pad_y, cut_loss, sub_
     """Drop-in for the loss block of ref_expert.py: `robust_loss = reproj_loss(prediction, gt_pose, f, padX, padY,
     opt.cutloss)` followed by `robust_loss.backward()`.  prediction [B,3,H,W] (CUDA), gt_poses [B,4,4] camera->world."""
     return ReprojLoss.apply(prediction, gt_poses, focal_length, pad_x, pad_y, cut_loss, sub_sampling, ppoint_x, ppoint_y)
+
+
+class InitLoss(torch.autograd.Function):
+    """init_expert.py:112-132 as one autograd node: forward = mean over the batch of the per-image scene-coordinate
+    losses, backward = their gradient, both from the single fused kernel behind api.init_loss.  The kernel returns the
+    gradient of each image's SUM; the 1/(B*count_b) of the two means is folded into the multiply by grad_out, with a scale
+    of 0 for an image without a valid cell (its loss is NaN, its gradient zero, as autograd gives the original)."""
+
+    @staticmethod
+    def forward(ctx, prediction, gt_coords, cut_loss):
+        grads = torch.empty_like(prediction)
+        res = api.init_loss(prediction.detach(), gt_coords, cut_loss, outGradients=grads)
+        B = len(res)
+        scale = torch.tensor([1.0 / (B * c) if c else 0.0 for _, c in res], dtype=prediction.dtype)
+        shape = (B, 1, 1, 1) if prediction.dim() == 4 else (1, 1, 1)
+        ctx.save_for_backward(grads, scale.view(shape).to(prediction.device))
+        return prediction.new_tensor(sum(l for l, _ in res) / B)
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        grads, scale = ctx.saved_tensors
+        return grads * (scale * grad_out), None, None
+
+
+def init_loss(prediction, gt_coords, cut_loss):
+    """Drop-in for the loss block of init_expert.py: `robust_loss = init_loss(prediction, gt_coords, opt.cutloss)`
+    followed by `robust_loss.backward()`, in place of util.assert_size through the division (:114-130).  prediction and
+    gt_coords [B,3,h,w] or [3,h,w] (sizes may differ by one pixel); returns the mean of the B per-image losses."""
+    return InitLoss.apply(prediction, gt_coords, cut_loss)

@@ -16,7 +16,7 @@ HERE = Path(__file__).resolve().parent
 CSRC = HERE / "csrc"
 OBJ = HERE / "_obj"
 LIB = HERE / "libesac_b200.so"
-SOURCES = ["score.cu", "hyp.cu", "refine.cu", "bwd.cu", "gating.cu", "reproj.cu", "capi.cu"]
+SOURCES = ["score.cu", "hyp.cu", "refine.cu", "bwd.cu", "gating.cu", "reproj.cu", "initloss.cu", "capi.cu"]
 HEADERS = ["esac_internal.h", "esac_geom.cuh", "esac_rng.cuh", "esac_p3p_fast.cuh", "../../include/esac_b200.h",
            "../../include/esac_b200_testhooks.h"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

@@ -1500,6 +1500,64 @@ int esacb200_reproj_loss(esacb200_ctx* ctx, int B, const float* coords, float* g
     return ESACB200_OK;
 } ESAC_ABI_CATCH(ctx)
 
+int esacb200_init_loss(esacb200_ctx* ctx, int B, const float* pred, int pred_H, int pred_W, const float* gt, int gt_H,
+                       int gt_W, float* grads, float cutLoss, double* out_sums, int64_t* out_counts) try {
+    if (!ctx) return ESACB200_ERR_ARG;
+    DeviceGuard device_guard(ctx->device);
+    if (!pred || !gt || !out_sums || !out_counts) return fail(ctx, ESACB200_ERR_ARG, "null pointer argument");
+    if (B <= 0 || B > 65535 || pred_H <= 0 || pred_W <= 0 || gt_H <= 0 || gt_W <= 0)
+        return fail(ctx, ESACB200_ERR_ARG, "bad sizes B=%d pred %dx%d gt %dx%d", B, pred_H, pred_W, gt_H, gt_W);
+    if (abs(pred_H - gt_H) > 1 || abs(pred_W - gt_W) > 1)   // util.assert_size
+        return fail(ctx, ESACB200_ERR_ARG, "Tensor size mismatch: prediction %dx%d, ground truth %dx%d (tolerance 1 px)",
+                    pred_H, pred_W, gt_H, gt_W);
+    if ((long long)pred_H * pred_W > (1ll << 30) || (long long)gt_H * gt_W > (1ll << 30))
+        return fail(ctx, ESACB200_ERR_ARG, "map too large");
+    begin_call(ctx);
+    const size_t pbytes = (size_t)B * 3 * pred_H * pred_W * sizeof(float), gbytes = (size_t)B * 3 * gt_H * gt_W * sizeof(float);
+    const bool p_host = !is_device_ptr(pred), t_host = !is_device_ptr(gt), g_host = grads && !is_device_ptr(grads);
+    const float* d_pred = pred;
+    const float* d_gt = gt;
+    float* d_grads = grads;
+    if (p_host) {
+        CK(ctx->coords.ensure(pbytes));
+        CK(cudaMemcpyAsync(ctx->coords.p, pred, pbytes, cudaMemcpyHostToDevice, ctx->stream));
+        d_pred = ctx->coords.as<float>();
+    }
+    if (t_host) {
+        CK(ctx->coords_alt.ensure(gbytes));
+        CK(cudaMemcpyAsync(ctx->coords_alt.p, gt, gbytes, cudaMemcpyHostToDevice, ctx->stream));
+        d_gt = ctx->coords_alt.as<float>();
+    }
+    if (g_host) {
+        CK(ctx->grads.ensure(pbytes));
+        d_grads = ctx->grads.as<float>();
+    }
+    const int bpi = init_loss_blocks_per_image(pred_H * pred_W);
+    // scratch layout: [tickets B u32, padded] [sums B f64] [counts B i64] [partial sums B*bpi f64] [partial counts B*bpi u32]
+    const size_t pad = 63, off_sum = ((size_t)B * 4 + pad) & ~pad, off_cnt = off_sum + (((size_t)B * 8 + pad) & ~pad),
+                 off_psum = off_cnt + (((size_t)B * 8 + pad) & ~pad), off_pcnt = off_psum + (((size_t)B * bpi * 8 + pad) & ~pad);
+    CK(ctx->scratch.ensure(off_pcnt + (size_t)B * bpi * 4));
+    char* base = (char*)ctx->scratch.p;
+    CK(cudaMemsetAsync(base, 0, off_sum, ctx->stream));
+    mark(ctx, EV_H2D);
+    mark(ctx, EV_FOLD);  // ms_score = the kernel alone
+    launch_init_loss(d_pred, d_gt, d_grads, B, pred_H, pred_W, gt_H, gt_W, cutLoss, bpi, (double*)(base + off_psum),
+                     (unsigned*)(base + off_pcnt), (unsigned*)base, (double*)(base + off_sum), (long long*)(base + off_cnt),
+                     ctx->stream);
+    CK(cudaGetLastError());
+    ctx->st.kernel_launches += 1;
+    mark(ctx, EV_SCORE);
+    if (g_host) CK(cudaMemcpyAsync(grads, d_grads, pbytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(out_sums, base + off_sum, (size_t)B * 8, cudaMemcpyDefault, ctx->stream));
+    CK(cudaMemcpyAsync(out_counts, base + off_cnt, (size_t)B * 8, cudaMemcpyDefault, ctx->stream));
+    mark(ctx, EV_END);
+    CK(cudaStreamSynchronize(ctx->stream));
+    CK(cudaGetLastError());
+    ctx->last_M = 0;
+    finish_stats(ctx);
+    return ESACB200_OK;
+} ESAC_ABI_CATCH(ctx)
+
 int esacb200_copy_last_scores(esacb200_ctx* ctx, double* dst, int M) try {
     if (!ctx || !dst) return ESACB200_ERR_ARG;
     DeviceGuard device_guard(ctx->device);

@@ -175,6 +175,14 @@ void launch_reproj(const float* coords, float* grads, const float* img, int B, i
                    float cy, float cut, float max_err, float min_depth, int blocks_per_image, double* partial,
                    unsigned* tickets, double* losses, cudaStream_t stream);
 
+// --- initloss.cu --------------------------------------------------------------------------
+int init_loss_blocks_per_image(int N);
+// pred / grads [B,3,pH,pW], gt [B,3,gH,gW] (|pH-gH|, |pW-gW| <= 1; the common top-left region counts), grads may be null.
+// partial_sum / partial_cnt: B * blocks_per_image each, tickets: B zeroed counters (left zeroed), sums / counts: B each.
+void launch_init_loss(const float* pred, const float* gt, float* grads, int B, int pH, int pW, int gH, int gW, float cut,
+                      int blocks_per_image, double* partial_sum, unsigned* partial_cnt, unsigned* tickets, double* sums,
+                      long long* counts, cudaStream_t stream);
+
 // --- bwd.cu -------------------------------------------------------------------------------
 struct BwdArgs {
     const float* coords;

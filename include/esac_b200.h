@@ -179,6 +179,21 @@ int esacb200_reproj_loss(esacb200_ctx* ctx, int B, const float* coords, float* g
                          const int* shiftX, const int* shiftY, float focalLength, float ppointX, float ppointY,
                          int subSampling, float cutLoss, float maxReproj, float minDepth, double* out_losses);
 
+/* Scene-coordinate loss of the expert initialisation stage and its gradient, one fused pass (init_expert.py:112-132,
+ * where it is about ten torch ops, two of them boolean-mask gathers, + autograd): pred float32 [B,3,pred_H,pred_W] and gt
+ * float32 [B,3,gt_H,gt_W], each contiguous at its own size; like util.assert_size both are cropped top-left to
+ * (min H, min W) (strides, no copy) and sizes that differ by more than 1 in either direction are an error.  A cell is valid
+ * where any gt component is nonzero (NaN included); d = ||pred - gt||; per image
+ *   out_sums[b]   = sum over valid cells of (d <= cutLoss ? d : sqrt(cutLoss * d))   (NaN d in neither branch)
+ *   out_counts[b] = number of valid cells (NaN d included)
+ * so init_expert.py's loss is out_sums[b] / out_counts[b] (NaN for an image without valid cells, as 0/0.0 in the reference).
+ * grads float32 [B,3,pred_H,pred_W] or NULL = d out_sums[b] / d pred -- the gradient of the SUM, not of the mean: scale by
+ * 1/out_counts[b] (overwritten, not accumulated; 0 for invalid and cropped-away cells and where d == 0, NaN where d is
+ * NaN).  out_sums host double [B], out_counts host int64 [B].  fp32 cell arithmetic like the original, fp64 sums in a
+ * fixed order: repeated calls are bit-identical. */
+int esacb200_init_loss(esacb200_ctx* ctx, int B, const float* pred, int pred_H, int pred_W, const float* gt, int gt_H,
+                       int gt_W, float* grads, float cutLoss, double* out_sums, int64_t* out_counts);
+
 /* Soft-inlier scores of given poses (getReproErrs + getHypScores, esac_util.h:235-363) without
  * sampling/selection/refinement: poses6 = host double [M][6] (rvec, tvec); out_scores host double [M]. */
 int esacb200_score_poses(esacb200_ctx* ctx, const float* coords, int E, int H, int W, const int64_t* assign,
